@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # B200 arm (this repo's CUDA path)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference algorithm on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # B200 arm, then DIR/*.npy: outputs of the last timed step
 
 One "step" = one evaluation of E[n] and dE/dn for the full kinetic functional WangGovindCarter99
 (TF + vW + non-local term, kernel cached) on the synthetic 256-atom Al supercell density of
@@ -43,6 +44,8 @@ N_FFT = 14
 # run (a run under ncu is never a bench value): per launch of the dominant stage, and summed over one evaluation
 NCU_TRAFFIC_256 = {'x-fwd * kernel-mix * x-inv (3 fields)': 0.9278e9, 'evaluation': 8.936e9}
 NCU_TRAFFIC_SOURCE = 'profiles/r02_ncu_full_wgc99_256_final.md (ncu --set full of one evaluation; not measured in this run)'
+DUMP_POINTS = 1 << 22          # grid points of dE/dn written by --dump-outputs: 32 MB of float64
+DUMP_SEED = 0
 
 
 def workload_config():
@@ -397,6 +400,8 @@ def run_gpu(args):
                         'launches': int(lib.pad_launch_count() - l0), 'fft_execs': int(lib.pad_fft_exec_count() - f0),
                         'caps': gc1[0] - gc0[0], 'reps': gc1[1] - gc0[1]})
         sampler = ClockSampler(local)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, E, g)
     pick = sorted(range(3), key=lambda i: regions[i]['ms_total'])[1]
     R = regions[pick]
     graph_caps_timed, graph_reps_timed = R['caps'], R['reps']
@@ -580,6 +585,22 @@ def run_gpu(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, E, g):
+    """--dump-outputs: what the last timed step handed its caller, as float64 .npy files, so that two builds can be compared
+    output for output.  energy.npy is E (Ha); grad_sample.npy is dE/dn (the autograd gradient with respect to the density) at
+    DUMP_POINTS grid points drawn with a fixed seed, in ascending flat (C-order) index -- the whole field if the grid is smaller
+    (at 256^3 the field alone is 128 MB)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = g.detach().reshape(-1)
+    if flat.numel() > DUMP_POINTS:
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(DUMP_SEED))[:DUMP_POINTS].sort().values
+        flat = flat[idx.to(flat.device)]
+    np.save(os.path.join(out_dir, 'energy.npy'), np.array([E.item()], dtype=np.float64))
+    np.save(os.path.join(out_dir, 'grad_sample.npy'), flat.double().cpu().numpy())
 
 
 def also_reported(dev, box, den):
@@ -972,7 +993,8 @@ class CleanStdout:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=50)
+    ap.add_argument('--steps', type=int, default=50,
+                    help='evaluations in each timed region (three regions back to back, the median one is reported)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
@@ -982,7 +1004,13 @@ def main():
                     help='functional evaluated in --slab-grid mode')
     ap.add_argument('--slab-grid', type=int, default=0,
                     help='strong-scaling mode: ONE n^3 grid slab-decomposed over the --gpus ranks (e.g. 512)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one returned (energy, seeded sample of dE/dn) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.slab_grid):
+        ap.error('--dump-outputs writes the outputs of the headline B200 run only')
     with CleanStdout():
         if args.impl == 'reference':
             run_reference(args)

@@ -251,6 +251,27 @@ def test_bench_helpers():
     assert bench.stage_bytes('y-fwd (4 fields)', 256 ** 3, ns) == 2 * 4 * 16 * ns
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: float64 .npy files within 64 MB at the headline size; a field larger than the sample is sampled at
+    the same seeded points every time, a smaller one is written whole."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert 8 * bench.DUMP_POINTS + 8 <= 64 * 2 ** 20 and bench.DUMP_POINTS < 256 ** 3
+    monkeypatch.setattr(bench, 'DUMP_POINTS', 500)
+    E = torch.tensor(-12.5, dtype=torch.double)
+    g = torch.rand(10, 11, 12, dtype=torch.double, generator=torch.Generator().manual_seed(1))
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), E, g)
+    a, b = (np.load(tmp_path / run / 'grad_sample.npy') for run in ('a', 'b'))
+    assert a.dtype == np.float64 and a.shape == (500,) and np.array_equal(a, b)
+    assert np.isin(a, g.numpy().ravel()).all() and len(np.unique(a)) == 500
+    assert np.load(tmp_path / 'a' / 'energy.npy').tolist() == [-12.5]
+    bench.dump_outputs(str(tmp_path / 'whole'), E, g[:5, :6, :7])
+    assert np.array_equal(np.load(tmp_path / 'whole' / 'grad_sample.npy'), g[:5, :6, :7].numpy().ravel())
+
+
 def test_elastic_averages_and_crystal_constructors():
     """elastic_tools.py:80-176 on the published Al XWM constants (docs/source/example_elastic.rst:161-178:
     C11/C12/C44 = 107.08 / 61.215 / 37.861 GPa) and the identities an isotropic medium must satisfy;
