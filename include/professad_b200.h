@@ -161,6 +161,14 @@ int pad_eval_wgc99(pad_plan* plan, const double* den, double alpha, double beta,
                    double* E_out, double* v_out, int accumulate, void* stream);
 /* PerdewBurkeErnzerhof (functionals.py:1597-1635); `which`: 1 = exchange, 2 = correlation, 3 = both */
 int pad_eval_pbe(pad_plan* plan, const double* den, int which, double* E_out, double* v_out, int accumulate, void* stream);
+/* Semilocal kinetic functionals T = int C_TF n^(5/3) F(p, q), p = s^2, q the reduced Laplacian (functional_tools.py:122-135):
+ *   PAD_SEMILOCAL_LKT  LuoKarasievTrickey (functionals.py:309):  F = 1/cosh(p0 s) + (5/3) p            (a = p0 = 1.3)
+ *   PAD_SEMILOCAL_PG   PauliGaussian      (functionals.py:336):  F = (5/3) p + exp(-p0 p) + p1 q^2     (mu = 40/27, beta = 0.25)
+ * Potential e_n - div(2 e_sigma grad n) + lap(e_L) from one gradient (and Laplacian) and one divergence round trip. */
+#define PAD_SEMILOCAL_LKT 0
+#define PAD_SEMILOCAL_PG 1
+int pad_eval_semilocal_kinetic(pad_plan* plan, const double* den, int variant, double p0, double p1, double* E_out, double* v_out,
+                               int accumulate, void* stream);
 
 /* HuangCarter.forward (variant 0: p0 = lambda) / RevisedHuangCarter.forward (variant 1: p0 = a, p1 = b)
  * (functionals.py:1232-1269, 1331-1365) with field_dependent_convolution + interpolate_kernel +
@@ -241,7 +249,8 @@ typedef struct pad_terms {
     int local_mask;      /* PAD_LOCAL_* bits (IonElectron needs v_ext)                       */
     int hartree;         /* 0/1                                                              */
     int kinetic;         /* 0 none, 1 Wang-Teter family (alpha, beta, kinetic_parts), 2 WGC99,
-                            3 Huang-Carter family (hc_* below; beta, kappa from the shared fields)      */
+                            3 Huang-Carter family (hc_* below; beta, kappa from the shared fields),
+                            4 semilocal (sl_* at the end; with pbe set both share one gradient / divergence round trip) */
     int kinetic_parts;   /* PAD_PART_* mask for kinetic == 1 (e.g. PAD_PART_VW alone = Weizsaecker) */
     int pbe;             /* 0 none, 1 exchange, 2 correlation, 3 both                        */
     double alpha, beta, gamma, kappa;
@@ -251,6 +260,9 @@ typedef struct pad_terms {
     int hc_n_eta;
     double hc_p0, hc_p1;
     const double* hc_table_dev;  /* DEVICE, 2 * hc_n_eta doubles [eta | omega(eta)]                             */
+    /* kinetic == 4: arguments of pad_eval_semilocal_kinetic */
+    int sl_variant;              /* PAD_SEMILOCAL_LKT or PAD_SEMILOCAL_PG                                      */
+    double sl_p0, sl_p1;
 } pad_terms;
 int pad_eval_total(pad_plan* plan, const pad_terms* terms, const double* den, const double* v_ext,
                    double* E_out, double* v_out, void* stream);
@@ -259,7 +271,8 @@ int pad_eval_total(pad_plan* plan, const pad_terms* terms, const double* den, co
  * IonElectron, see pad_ion_stress): replaces get_stress / System.__compute_stress (functional_tools.py:73-100,
  * system.py:927-935; formulas tests/tools_for_tests.py:212-472).  stress_out: DEVICE, 9 doubles, overwritten.
  * Every kinetic kind is covered: Wang-Teter family, WangGovindCarter99 (kernel regenerated for the strained cell) and the
- * Huang-Carter family (xi-node list held fixed, as the reference's autograd sees it, functional_tools.py:408-416). */
+ * Huang-Carter family (xi-node list held fixed, as the reference's autograd sees it, functional_tools.py:408-416) and the
+ * semilocal kind (LuoKarasievTrickey, PauliGaussian: gradient and Laplacian terms). */
 int pad_stress_terms(pad_plan* plan, const pad_terms* terms, const double* den, double* stress_out, void* stream);
 
 /* ---- ion-ion interaction: replaces ion_interaction_sum (ion_utils.py:293-333; torch_nl pair list + autograd) with a

@@ -19,7 +19,8 @@ class PadTerms(ctypes.Structure):
                 ('alpha', ctypes.c_double), ('beta', ctypes.c_double), ('gamma', ctypes.c_double),
                 ('kappa', ctypes.c_double),
                 ('hc_variant', ctypes.c_int), ('hc_geometric', ctypes.c_int), ('hc_n_eta', ctypes.c_int),
-                ('hc_p0', ctypes.c_double), ('hc_p1', ctypes.c_double), ('hc_table_dev', ctypes.c_void_p)]
+                ('hc_p0', ctypes.c_double), ('hc_p1', ctypes.c_double), ('hc_table_dev', ctypes.c_void_p),
+                ('sl_variant', ctypes.c_int), ('sl_p0', ctypes.c_double), ('sl_p1', ctypes.c_double)]
 
 
 class PadDenoptParams(ctypes.Structure):
@@ -84,6 +85,11 @@ def describe_terms(terms, device=None):
             T.hc_n_eta = int(table.shape[1])
             T.hc_table_dev = table.data_ptr()
             T._keep = table             # the descriptor holds a raw device pointer: keep the tensor alive with it
+        elif kind == 'semilocal':
+            if T.kinetic:
+                return None
+            T.kinetic = 4
+            T.sl_variant, T.sl_p0, T.sl_p1 = spec[1:4]
         else:
             return None
     if not (T.local_mask or T.hartree or T.kinetic or T.pbe):

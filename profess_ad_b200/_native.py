@@ -44,6 +44,7 @@ SIGNATURES = {
     'pad_eval_wt_components': (_int, [_vp, _vp, _dbl, _dbl, _vp, _vp, _vp]),
     'pad_eval_wgc99': (_int, [_vp, _vp, _dbl, _dbl, _dbl, _dbl, _vp, _vp, _int, _vp]),
     'pad_eval_pbe': (_int, [_vp, _vp, _int, _vp, _vp, _int, _vp]),
+    'pad_eval_semilocal_kinetic': (_int, [_vp, _vp, _int, _dbl, _dbl, _vp, _vp, _int, _vp]),
     'pad_eval_hc': (_int, [_vp, _vp, _int, _dbl, _dbl, _dbl, _dbl, _int, _vp, _int, _vp, _vp, _int, _vp, _vp]),
     'pad_set_fast_fft': (_int, [_int]),
     'pad_set_option': (_int, [ctypes.c_char_p, _int]),
@@ -80,6 +81,7 @@ SIGNATURES = {
 
 PART_TF, PART_VW, PART_NL, PART_ALL = 1, 2, 4, 7
 LOCAL_TF, LOCAL_LDAX, LOCAL_PZC, LOCAL_IONEL = 1, 2, 4, 8
+SEMILOCAL_LKT, SEMILOCAL_PG = 0, 1
 
 _lib = None
 _lock = threading.Lock()

@@ -345,6 +345,19 @@ int pad_pbe_pointwise(pad_plan* p, cudaStream_t s, const double* den, double* gx
                       int accumulate, int* grid_out);
 int pad_pbe_fast_supported(const pad_plan* p);
 int pad_pbe_fast(pad_plan* p, const double* den, int which, double* E_out, double* v_out, int accumulate, cudaStream_t s);
+// semilocal kinetic functional (PAD_SEMILOCAL_*, parameters p0, p1) plus, with pbe != 0, the PBE terms (1 x, 2 c, 3 both) in the
+// same point kernel
+struct pad_semilocal_args {
+    int variant;
+    double p0, p1;
+    int pbe;
+};
+int pad_semilocal_pointwise(pad_plan* p, cudaStream_t s, const double* den, double* gx, double* gy, double* gz, double* lap, double* v,
+                            const pad_semilocal_args& P, int accumulate, int* grid_out);
+int pad_semilocal_fast(pad_plan* p, const double* den, const pad_semilocal_args& P, double* E_out, double* v_out, int accumulate,
+                       cudaStream_t s);
+int pad_eval_semilocal_ex(pad_plan* p, const double* den, const pad_semilocal_args& P, double* E_out, double* v_out, int accumulate,
+                          void* stream);
 int pad_hartree_fast_supported(const pad_plan* p);
 int pad_hartree_fast(pad_plan* p, const double* den, double* E_out, double* v_out, int accumulate, cudaStream_t s);
 int pad_wt_fast_supported(const pad_plan* p);

@@ -143,7 +143,7 @@ __device__ __forceinline__ void zfwd_field(const Gen& gen, const double (&sa)[Ge
 //   gen.stage(in[NIN] (double2 each: the points g, g + 1), a[NST], b[NST])
 //   gen.field<F>(st[NST])           value of field F at a point
 struct ZIn {
-    const double* f[3];
+    const double* f[4];
 };
 
 template <int M, int TPL, int NF, class Gen>
@@ -561,7 +561,7 @@ inline int z_lines(const pad_plan* p) { return (p->dist ? p->n0_loc : p->n0) * p
 
 template <int M, int TPL, int NF, class Gen>
 int launch_zfwd(pad_plan* p, cudaStream_t s, Gen gen, const double* in0, const double* in1, cd* o0, cd* o1, cd* o2, cd* o3,
-                const double* in2 = nullptr) {
+                const double* in2 = nullptr, const double* in3 = nullptr) {
     constexpr int warps = 4;
     using L = ZLayout<M, TPL>;
     constexpr int smem = L::kTwBytes + warps * L::kLinesPerWarp * L::fwd_line_bytes(Gen::NIN);
@@ -572,7 +572,7 @@ int launch_zfwd(pad_plan* p, cudaStream_t s, Gen gen, const double* in0, const d
         attr_done[p->device & 63] = true;
     }
     const int nlines = z_lines(p);
-    ZIn in{{in0, in1, in2}};
+    ZIn in{{in0, in1, in2, in3}};
     kern<<<zgrid(nlines, warps * (32 / TPL), 4), warps * 32, smem, s>>>(gen, in, o0, o1, o2, o3, nlines, p->nzp);
     ++g_pad_launches;
     PAD_CUDA(cudaGetLastError());
@@ -783,7 +783,7 @@ int launch_zy_fwd_L(pad_plan* p, cudaStream_t s, Gen gen, const double* in0, con
     sh.items[2] = 0;
     constexpr int by_smem = (227 * 1024) / (smem + 1024);
     const int grid = 148 * (by_smem < 4 ? by_smem : 4);
-    ZIn in{{in0, in1, nullptr}};
+    ZIn in{{in0, in1, nullptr, nullptr}};
     SPassFields o;
     for (int i = 0; i < 4; ++i) o.f[i] = i < NF ? out[i] : nullptr;
     kern<<<grid, warps * 32, smem, s>>>(gen, in, o, reinterpret_cast<PipeCtl*>(p->pipe_ctl), sh, g);
@@ -1122,18 +1122,21 @@ int launch_xmix_L(pad_plan* p, cudaStream_t s, const SPassFields& f, const SPass
     return PAD_OK;
 }
 
-// gradient (NIN = 1: one spectrum in, three out) and divergence (NOUT = 1: three in, one out) forms of the fused x pass
-template <int NIN, int NOUT, class Mix>
+// gradient (NIN = 1: one spectrum in, NF out) and divergence (NOUT = 1: NF in, one out) forms of the fused x pass;
+// NF = 3: grad / div, NF = 4 (n0 <= 256): grad and Laplacian / div and Laplacian (semilocal functionals of lap n)
+template <int NIN, int NOUT, class Mix, int NF = 3>
 int launch_xmix3_io(pad_plan* p, cudaStream_t s, cd* const* fields, Mix mix) {
     if (p->dist) { pad_set_error("fused x pass (gradient / divergence form): single-GPU plans only"); return PAD_ERR_ARG; }
     SPassFields f;
-    for (int i = 0; i < 4; ++i) f.f[i] = i < 3 ? fields[i] : nullptr;
+    for (int i = 0; i < 4; ++i) f.f[i] = i < NF ? fields[i] : nullptr;
     const SPassGeom g = spass_geom(p, 0);
     switch (p->n0) {
-        case 64: return launch_xmix_L<64, 3, Mix, false, NIN, NOUT>(p, s, f, g, mix);
-        case 128: return launch_xmix_L<128, 3, Mix, false, NIN, NOUT>(p, s, f, g, mix);
-        case 256: return launch_xmix_L<256, 3, Mix, false, NIN, NOUT>(p, s, f, g, mix);
-        case 512: return launch_xmix_L<512, 3, Mix, false, NIN, NOUT>(p, s, f, g, mix);
+        case 64: return launch_xmix_L<64, NF, Mix, false, NIN, NOUT>(p, s, f, g, mix);
+        case 128: return launch_xmix_L<128, NF, Mix, false, NIN, NOUT>(p, s, f, g, mix);
+        case 256: return launch_xmix_L<256, NF, Mix, false, NIN, NOUT>(p, s, f, g, mix);
+        case 512:
+            if constexpr (NF <= 3) return launch_xmix_L<512, NF, Mix, false, NIN, NOUT>(p, s, f, g, mix);
+            break;              // four 512-point tiles do not fit in shared memory: the caller takes the cuFFT route
     }
     pad_set_error("fused x pass: length %d not supported", p->n0);
     return PAD_ERR_ARG;
@@ -2867,6 +2870,205 @@ int pad_pbe_fast(pad_plan* p, const double* den, int which, double* E_out, doubl
     pad_stage_mark("PBE: y-inv", s);
     ZDISPATCH(p, PAD_TRY((launch_zinv<M, TPL, 1, 0>(p, s, PostPbeDiv{v_out}, B[0], nullptr, nullptr, nullptr, nullptr, v_out, nullptr))));
     pad_stage_mark("PBE: z-c2r + v -= div w", s);
+    return PAD_OK;
+}
+
+// =================================================================================================
+//  Semilocal kinetic functionals (LuoKarasievTrickey, PauliGaussian: xc.cuh, semilocal_kinetic_point), optionally with PBE
+//  in the same point kernel (pad_eval_total: one gradient / divergence round trip carries both energy densities and both w)
+//     LKT: the PBE passes.  PG (depends on L = lap n): the x passes carry a fourth field,
+//       [x . (i k_c / N, -k^2 / N) . x^-1: one in, four out]  ...  [x . (i k . w + k^2 e_L) / N . x^-1: four in, one out]
+//     so that v = e_n - div(2 e_sigma grad n) + lap(e_L) comes out of the same single-field tail.
+//  -k^2 is the Hermitian part (sym_even) on the special points, as in pad_laplacian.
+// =================================================================================================
+struct MixGradLapCoef {
+    double kx, ky, kz, k2;
+};
+struct MixGradLap {                    // q[0] = F  ->  q[c] = i k_c F / N (c < 3), q[3] = -k^2 F / N
+    static constexpr int kRing = 1;
+    double inv_n;
+    typedef MixGradLapCoef Coef;
+    typedef MixGrad::Line Line;
+    __device__ __forceinline__ Line line(const KGeom& g, int ky, int z) const { return Line{&g, ky, z}; }
+    __device__ __forceinline__ Coef fetch(const Line& l, int kx, size_t, bool live) const {
+        Coef c{0.0, 0.0, 0.0, 0.0};
+        if (live) {
+            const KPoint p = make_kpoint_at(*l.g, kx, l.ky, l.z);
+            sym_kvec(p, c.kx, c.ky, c.kz);
+            c.kx *= inv_n; c.ky *= inv_n; c.kz *= inv_n;
+            c.k2 = inv_n * sym_even(p, [](double x, double y, double z) { return x * x + y * y + z * z; });
+        }
+        return c;
+    }
+    __device__ __forceinline__ void apply(const Coef& k, cd* q) const {
+        const cd a = q[0];
+        q[0] = cd{-a.y * k.kx, a.x * k.kx};
+        q[1] = cd{-a.y * k.ky, a.x * k.ky};
+        q[2] = cd{-a.y * k.kz, a.x * k.kz};
+        q[3] = cd{-a.x * k.k2, -a.y * k.k2};
+    }
+};
+struct MixDivLap {                     // q[0] = (i k . (q0, q1, q2) + k^2 q3) / N  (the tail subtracts it from v)
+    static constexpr int kRing = 1;
+    double inv_n;
+    typedef MixGradLapCoef Coef;
+    typedef MixGrad::Line Line;
+    __device__ __forceinline__ Line line(const KGeom& g, int ky, int z) const { return Line{&g, ky, z}; }
+    __device__ __forceinline__ Coef fetch(const Line& l, int kx, size_t pidx, bool live) const { return MixGradLap{inv_n}.fetch(l, kx, pidx, live); }
+    __device__ __forceinline__ void apply(const Coef& k, cd* q) const {
+        const double re = k.kx * q[0].x + k.ky * q[1].x + k.kz * q[2].x, im = k.kx * q[0].y + k.ky * q[1].y + k.kz * q[2].y;
+        q[0] = cd{-im + k.k2 * q[3].x, re + k.k2 * q[3].y};
+    }
+};
+struct PostStore4 {                    // plain c2r of four real fields
+    static constexpr bool kDen = false, kVin = false;
+    static constexpr int NST = 0;
+    double *o0, *o1, *o2, *o3;
+    __device__ void apply(size_t g, double2, double2, const double* u0, const double* u1, double*, double*, double*) const {
+        *reinterpret_cast<double2*>(o0 + g) = make_double2(u0[0], u1[0]);
+        *reinterpret_cast<double2*>(o1 + g) = make_double2(u0[1], u1[1]);
+        *reinterpret_cast<double2*>(o2 + g) = make_double2(u0[2], u1[2]);
+        *reinterpret_cast<double2*>(o3 + g) = make_double2(u0[3], u1[3]);
+    }
+    static constexpr int NACC = 0;
+    typedef int Ctx;
+    __device__ Ctx begin() const { return 0; }
+    template <int F>
+    __device__ void fold(const Ctx&, double, double, double*) const {}
+    __device__ void finish(const Ctx&, size_t, double2, const double*, const double*, double, double, double*, double*, double*) const {}
+};
+struct GenCopy4 {                      // plain r2c of four real fields
+    static constexpr int NST = 4, NIN = 4;
+    __device__ void stage(const double2* in, double* a, double* b) const {
+        a[0] = in[0].x; a[1] = in[1].x; a[2] = in[2].x; a[3] = in[3].x;
+        b[0] = in[0].y; b[1] = in[1].y; b[2] = in[2].y; b[3] = in[3].y;
+    }
+    template <int F>
+    __device__ double field(const double* s) const { return s[F]; }
+};
+
+// semilocal_kinetic_point (xc.cuh) with the table log / exp of fastmath.cuh: one log of n and two exps give n^(2/3) and
+// n^(-8/3); LKT adds exp(-a s) (1/cosh and tanh from it: 2 e^-x / (1 + e^-2x) cannot overflow), PG exp(-mu p).  Arguments
+// outside the fast range take the library version.
+__device__ __forceinline__ void semilocal_kinetic_point_fast(double n, double sig, double lap, int variant, double p0, double p1,
+                                                             double& e, double& e_n, double& e_sig, double& e_lap) {
+    if (!(n > 1e-20 && n < 1e20 && sig < 1e40 && fabs(lap) < 1e40)) {
+        semilocal_kinetic_point(n, sig, lap, variant, p0, p1, e, e_n, e_sig, e_lap);
+        return;
+    }
+    const double l = fm_log(n);
+    const double n23 = fm_exp((2.0 / 3.0) * l), im83 = fm_exp((-8.0 / 3.0) * l);      // n^(2/3), n^(-8/3)
+    const double p = kSlC * sig * im83;
+    double F, Fp, qFq = 0.0;
+    e_lap = 0.0;
+    if (variant == 0) {
+        const double x = p0 * sqrt(p);
+        const double em = fm_exp(-fmin(x, 300.0)), em2 = em * em;                       // e^-x (e^-300: sech below 1e-130)
+        const double ir = fm_recip(1.0 + em2);
+        const double sech = 2.0 * em * ir;
+        const double tox = x < 0.0625 ? tanh_over_x_series(x) : (1.0 - em2) * ir * fm_recip(x);
+        F = sech + (5.0 / 3.0) * p;
+        Fp = 5.0 / 3.0 - 0.5 * p0 * p0 * sech * tox;
+    } else {
+        const double q = kSlC * lap * (n * im83), g = fm_exp(-fmin(p0 * p, 700.0));
+        F = (5.0 / 3.0) * p + g + p1 * q * q;
+        Fp = 5.0 / 3.0 - p0 * g;
+        qFq = 2.0 * p1 * q * q;
+        e_lap = kCTF * kSlC * 2.0 * p1 * q;
+    }
+    e = kCTF * n * n23 * F;
+    e_n = kCTF * n23 * ((5.0 / 3.0) * F - (8.0 / 3.0) * p * Fp - (5.0 / 3.0) * qFq);
+    e_sig = kCTF * kSlC * Fp * fm_recip(n);
+}
+
+// n, grad n (, lap n) -> energy density (one block-reduced sum), v (+)= e_n, grad n <- w = 2 e_sigma grad n (, lap n <- e_L);
+// with P.pbe the PBE terms are added to e, e_n, e_sigma at the same point.  Plain one-point-per-thread loads: any alignment,
+// any N (the cuFFT route takes odd grids and caller-owned pointers)
+template <bool LAP>
+__global__ void __launch_bounds__(PAD_THREADS) semilocal_point_kernel(const double* __restrict__ den, double* __restrict__ gx,
+                                                                     double* __restrict__ gy, double* __restrict__ gz,
+                                                                     double* __restrict__ lap, double* __restrict__ v, size_t n,
+                                                                     pad_semilocal_args P, int accumulate,
+                                                                     double* __restrict__ partials) {
+    fm_load_tables();
+    double acc[1] = {0.0};
+    const size_t stride = (size_t)gridDim.x * PAD_THREADS;
+    for (size_t i = (size_t)blockIdx.x * PAD_THREADS + threadIdx.x; i < n; i += stride) {
+        const double d = den[i], x = gx[i], y = gy[i], z = gz[i];
+        const double sig = x * x + y * y + z * z;
+        double e, e_n, e_s, e_l;
+        semilocal_kinetic_point_fast(d, sig, LAP ? lap[i] : 0.0, P.variant, P.p0, P.p1, e, e_n, e_s, e_l);
+        if (P.pbe) {
+            double f, f_n, f_s;
+            pbe_point_fast(d, sig, (P.pbe & 1) != 0, (P.pbe & 2) != 0, f, f_n, f_s);
+            e += f; e_n += f_n; e_s += f_s;
+        }
+        acc[0] += e;
+        if (v) {
+            v[i] = (accumulate ? v[i] : 0.0) + e_n;
+            const double w = 2.0 * e_s;
+            gx[i] = w * x; gy[i] = w * y; gz[i] = w * z;
+            if (LAP) lap[i] = e_l;
+        }
+    }
+    block_reduce_store<1>(acc, partials);
+}
+
+int pad_semilocal_pointwise(pad_plan* p, cudaStream_t s, const double* den, double* gx, double* gy, double* gz, double* lap, double* v,
+                            const pad_semilocal_args& P, int accumulate, int* grid_out) {
+    PAD_TRY(ensure_twiddles(p->device));
+    const int grid = pad_grid_for(p->N);
+    if (lap) semilocal_point_kernel<true><<<grid, PAD_THREADS, 0, s>>>(den, gx, gy, gz, lap, v, p->N, P, accumulate, p->partials);
+    else semilocal_point_kernel<false><<<grid, PAD_THREADS, 0, s>>>(den, gx, gy, gz, nullptr, v, p->N, P, accumulate, p->partials);
+    ++g_pad_launches;
+    PAD_CUDA(cudaGetLastError());
+    if (grid_out) *grid_out = grid;
+    return PAD_OK;
+}
+
+int pad_semilocal_fast(pad_plan* p, const double* den, const pad_semilocal_args& P, double* E_out, double* v_out, int accumulate,
+                       cudaStream_t s) {
+    PAD_TRY(ensure_twiddles(p->device));
+    const bool lap = P.variant == PAD_SEMILOCAL_PG;
+    const int nf = lap ? 4 : 3;
+    cd* B[4];
+    double* G[4];
+    for (int i = 0; i < nf; ++i) { PAD_TRY(get_zbuf(p, i, &B[i])); PAD_TRY(pad_get_rbuf(p, i, &G[i])); }
+    const double inv_n = p->geom.inv_n;
+    pad_stage_begin(s);
+    ZDISPATCH(p, PAD_TRY((launch_zfwd<M, TPL, 1>(p, s, GenCopy{}, den, nullptr, B[0], nullptr, nullptr, nullptr))));
+    pad_stage_mark("semilocal: z-r2c", s);
+    PAD_TRY(launch_spass(p, s, 1, -1, B, 1));
+    pad_stage_mark("semilocal: y-fwd", s);
+    if (lap) PAD_TRY((launch_xmix3_io<1, 4, MixGradLap, 4>(p, s, B, MixGradLap{inv_n})));
+    else PAD_TRY((launch_xmix3_io<1, 3>(p, s, B, MixGrad{inv_n})));
+    pad_stage_mark("semilocal: x-fwd * (i k [, -k^2]) * x-inv (1 -> 3 | 4)", s);
+    PAD_TRY(launch_spass(p, s, 1, +1, B, nf));
+    pad_stage_mark("semilocal: y-inv (3 | 4)", s);
+    if (lap) ZDISPATCH(p, PAD_TRY((launch_zinv<M, TPL, 4, 0>(p, s, PostStore4{G[0], G[1], G[2], G[3]}, B[0], B[1], B[2], B[3], nullptr, nullptr, nullptr))));
+    else ZDISPATCH(p, PAD_TRY((launch_zinv<M, TPL, 3, 0>(p, s, PostStore3{G[0], G[1], G[2]}, B[0], B[1], B[2], nullptr, nullptr, nullptr, nullptr))));
+    pad_stage_mark("semilocal: z-c2r (3 | 4)", s);
+    int grid = 1;
+    PAD_TRY(pad_semilocal_pointwise(p, s, den, G[0], G[1], G[2], lap ? G[3] : nullptr, v_out, P, accumulate, &grid));
+    pad_stage_mark("semilocal: energy density, e_n, w [, e_L] (pointwise)", s);
+    if (E_out) {
+        FinalizeArgs a = wgc_energy_args(p, grid, 1, accumulate, E_out);
+        a.coef[0] = p->dV;
+        pad_launch_finalize(p, a, s);
+    }
+    if (!v_out) return PAD_OK;
+    if (lap) ZDISPATCH(p, PAD_TRY((launch_zfwd<M, TPL, 4>(p, s, GenCopy4{}, G[0], G[1], B[0], B[1], B[2], B[3], G[2], G[3]))));
+    else ZDISPATCH(p, PAD_TRY((launch_zfwd<M, TPL, 3>(p, s, GenCopy3{}, G[0], G[1], B[0], B[1], B[2], nullptr, G[2]))));
+    pad_stage_mark("semilocal: z-r2c (3 | 4)", s);
+    PAD_TRY(launch_spass(p, s, 1, -1, B, nf));
+    pad_stage_mark("semilocal: y-fwd (3 | 4)", s);
+    if (lap) PAD_TRY((launch_xmix3_io<4, 1, MixDivLap, 4>(p, s, B, MixDivLap{inv_n})));
+    else PAD_TRY((launch_xmix3_io<3, 1>(p, s, B, MixDiv{inv_n})));
+    pad_stage_mark("semilocal: x-fwd * (i k . [, k^2]) * x-inv (3 | 4 -> 1)", s);
+    PAD_TRY(launch_spass(p, s, 1, +1, B, 1));
+    pad_stage_mark("semilocal: y-inv", s);
+    ZDISPATCH(p, PAD_TRY((launch_zinv<M, TPL, 1, 0>(p, s, PostPbeDiv{v_out}, B[0], nullptr, nullptr, nullptr, nullptr, v_out, nullptr))));
+    pad_stage_mark("semilocal: z-c2r + v -= div w [- lap e_L]", s);
     return PAD_OK;
 }
 

@@ -989,3 +989,89 @@ extern "C" int pad_eval_pbe(pad_plan* p, const double* den, int which, double* E
     PAD_CHECK_LAUNCH();
     return PAD_OK;
 }
+
+// =============================================================================================
+//  Semilocal kinetic functionals (LuoKarasievTrickey functionals.py:309, PauliGaussian functionals.py:336), 8 FFTs
+//  (10 with the Laplacian).  Potential = e_n - div(2 e_sigma grad n) + lap(e_L); with P.pbe the PBE terms share the
+//  point kernel and both round trips (pad_eval_total).  Fused passes where pad_pbe_fast_supported holds (PG: and n0 <= 256),
+//  else cuFFT (any grid, slab plans).
+// =============================================================================================
+int pad_eval_semilocal_ex(pad_plan* p, const double* den, const pad_semilocal_args& P, double* E_out, double* v_out, int accumulate,
+                          void* stream) {
+    PAD_TRY(check_common(p, den, "pad_eval_semilocal_kinetic"));
+    if (P.variant != PAD_SEMILOCAL_LKT && P.variant != PAD_SEMILOCAL_PG) {
+        pad_set_error("pad_eval_semilocal_kinetic: variant must be PAD_SEMILOCAL_LKT (0) or PAD_SEMILOCAL_PG (1)");
+        return PAD_ERR_ARG;
+    }
+    cudaStream_t s = as_stream(stream);
+    if (g_pad_fast_fft && pad_pbe_fast_supported(p) && (P.variant != PAD_SEMILOCAL_PG || p->n0 <= 256) &&
+        ((reinterpret_cast<uintptr_t>(den) | reinterpret_cast<uintptr_t>(v_out)) & 15) == 0)
+        return pad_semilocal_fast(p, den, P, E_out, v_out, accumulate, s);
+    const bool lap = P.variant == PAD_SEMILOCAL_PG;
+    double* R[4];
+    cufftDoubleComplex* C[4];
+    for (int i = 0; i < 4; ++i) { PAD_TRY(pad_get_rbuf(p, i, &R[i])); PAD_TRY(pad_get_cbuf(p, i, &C[i])); }
+    PAD_TRY(pad_fft_forward(p, den, C[0], s));
+    const double inv_n = p->geom.inv_n;
+    {   // i k_c F / N -> C1..C3 and, for the Laplacian, -k^2 F / N in place in C0
+        cufftDoubleComplex *F = C[0], *Gx = C[1], *Gy = C[2], *Gz = C[3];
+        launch_ks(p, s, [=] __device__(uint32_t idx, const KPoint& k) {
+            double kx, ky, kz;
+            sym_kvec(k, kx, ky, kz);
+            const cufftDoubleComplex c = F[idx];
+            const double a = c.x * inv_n, b = c.y * inv_n;
+            Gx[idx] = make_cuDoubleComplex(-b * kx, a * kx);
+            Gy[idx] = make_cuDoubleComplex(-b * ky, a * ky);
+            Gz[idx] = make_cuDoubleComplex(-b * kz, a * kz);
+            if (lap) {
+                const double m = -sym_even(k, [](double x, double y, double z) { return x * x + y * y + z * z; });
+                F[idx] = make_cuDoubleComplex(m * a, m * b);
+            }
+        });
+        PAD_CHECK_LAUNCH();
+    }
+    cufftDoubleComplex* Cin[4] = {C[1], C[2], C[3], C[0]};
+    PAD_TRY(pad_fft_inverse_many(p, Cin, R, lap ? 4 : 3, s));
+    int grid = 0;
+    PAD_TRY(pad_semilocal_pointwise(p, s, den, R[0], R[1], R[2], lap ? R[3] : nullptr, v_out, P, accumulate, &grid));
+    if (E_out) {
+        FinalizeArgs a;
+        a.nblocks = grid; a.nterms = 1; a.accumulate = accumulate;
+        for (int t = 0; t < PAD_MAX_RED; ++t) a.coef[t] = 0.0;
+        a.coef[0] = p->dV;
+        a.sums_out = nullptr;
+        a.E_out = E_out;
+        pad_launch_finalize(p, a, s);
+    }
+    PAD_CHECK_LAUNCH();
+    if (!v_out) return PAD_OK;
+    PAD_TRY(pad_fft_forward_many(p, R, C, lap ? 4 : 3, s));
+    {   // (i k . w + k^2 e_L) / N -> C0
+        cufftDoubleComplex *C0 = C[0], *C1 = C[1], *C2 = C[2], *C3 = C[3];
+        launch_ks(p, s, [=] __device__(uint32_t idx, const KPoint& k) {
+            double kx, ky, kz;
+            sym_kvec(k, kx, ky, kz);
+            const cufftDoubleComplex a = C0[idx], b = C1[idx], c = C2[idx];
+            double re = kx * a.x + ky * b.x + kz * c.x, im = kx * a.y + ky * b.y + kz * c.y;
+            double xr = -im, xi = re;
+            if (lap) {
+                const double m = sym_even(k, [](double x, double y, double z) { return x * x + y * y + z * z; });
+                const cufftDoubleComplex l = C3[idx];
+                xr += m * l.x; xi += m * l.y;
+            }
+            C0[idx] = make_cuDoubleComplex(xr * inv_n, xi * inv_n);
+        });
+        PAD_CHECK_LAUNCH();
+    }
+    PAD_TRY(pad_fft_inverse(p, C[0], R[0], s));
+    const double* Dv = R[0];
+    launch_ew<0>(p, s, [=] __device__(size_t i, double(&)[1]) { v_out[i] -= Dv[i]; });
+    PAD_CHECK_LAUNCH();
+    return PAD_OK;
+}
+
+extern "C" int pad_eval_semilocal_kinetic(pad_plan* p, const double* den, int variant, double p0, double p1, double* E_out,
+                                          double* v_out, int accumulate, void* stream) {
+    const pad_semilocal_args P{variant, p0, p1, 0};
+    return pad_eval_semilocal_ex(p, den, P, E_out, v_out, accumulate, stream);
+}

@@ -455,8 +455,13 @@ extern "C" int pad_eval_total(pad_plan* p, const pad_terms* T, const double* den
         PAD_TRY(pad_eval_hc(p, den, T->hc_variant, T->hc_p0, T->hc_p1, T->beta, T->kappa, T->hc_geometric, T->hc_table_dev,
                             T->hc_n_eta, E_out, v_out, 1, nullptr, stream));
         acc = 1;
+    } else if (T->kinetic == 4) {
+        // PBE rides along: one gradient / divergence round trip carries both energy densities and both w fields
+        const pad_semilocal_args P{T->sl_variant, T->sl_p0, T->sl_p1, T->pbe};
+        PAD_TRY(pad_eval_semilocal_ex(p, den, P, E_out, v_out, acc, stream));
+        acc = 1;
     }
-    if (T->pbe) {
+    if (T->pbe && T->kinetic != 4) {
         PAD_TRY(pad_eval_pbe(p, den, T->pbe, E_out, v_out, acc, stream));
         acc = 1;
     }

@@ -11,6 +11,9 @@
 //   Weizsaecker             : - sum_k w |chi_k|^2 k_i k_j
 //   Wang-Teter family NL    : pref sum_k w Re(a_k conj b_k) aux3(eta) (k_i k_j / k^2 - delta_ij / 3) - (2/3) delta_ij T_NL / vol
 //   PBE                     : delta_ij mean(f - n f_n - 2 sigma f_sigma) - 2 mean(f_sigma g_i g_j)
+//   semilocal kinetic (LKT, PG): delta_ij mean(e - n e_n - 2 sigma e_sigma - L e_L) - 2 mean(e_sigma g_i g_j)
+//                             - 2 mean(e_L d_i d_j n),  the last as  2 sum_k w Re(conj(l_k) c_k) k_i k_j
+//                             (l_k: coefficients of e_L; the strain derivative of -k^2 is 2 k_i k_j with the same k)
 // (c_k, chi_k, a_k, b_k: Fourier coefficients, norm = 'forward', of n, sqrt n, n^alpha, n^beta.)
 //   WangGovindCarter99 NL   : pad_stress_wgc99_nl (functionals.cu): same structure with the eta-derivatives of the four kernels;
 //                             the derivative with the kernel regenerated for the strained cell (the reference's autograd
@@ -83,7 +86,7 @@ extern "C" int pad_stress_terms(pad_plan* p, const pad_terms* T, const double* d
     // ---- local terms (IonElectron is handled by pad_ion_stress) ------------------------------------------
     // WangGovindCarter99 = TF + vW + its own non-local term (functionals.py:983-985)
     // HuangCarter / RevisedHuangCarter = TF + vW + their non-local term too (functionals.py:1267-1269)
-    int parts = T->kinetic == 1 ? T->kinetic_parts : (T->kinetic >= 2 ? (PAD_PART_TF | PAD_PART_VW) : 0);
+    int parts = T->kinetic == 1 ? T->kinetic_parts : (T->kinetic == 2 || T->kinetic == 3 ? (PAD_PART_TF | PAD_PART_VW) : 0);
     // ThomasFermi can appear as a term of its own and inside a Wang-Teter style functional: count both
     const double tfc = ((T->local_mask & PAD_LOCAL_TF) ? 1.0 : 0.0) + ((parts & PAD_PART_TF) ? 1.0 : 0.0);
     const bool tf = tfc != 0.0;
@@ -206,6 +209,40 @@ extern "C" int pad_stress_terms(pad_plan* p, const pad_terms* T, const double* d
             add_tensor(acc, -2.0 * f_sig, gx, gy, gz);
         });
         PAD_TRY(pad_stress_accumulate(p, s, gN, inv_n, inv_n, stress_out));
+    }
+
+    // ---- semilocal kinetic functionals -------------------------------------------------------------------------------
+    if (T->kinetic == 4) {
+        const bool lap = T->sl_variant == PAD_SEMILOCAL_PG;
+        for (int i = 0; i < 4; ++i) PAD_TRY(pad_get_rbuf(p, i, &R[i]));
+        PAD_TRY(pad_gradient(p, den, R[0], R[1], R[2], stream));
+        if (lap) PAD_TRY(pad_laplacian(p, den, R[3], stream));
+        const double *Gx = R[0], *Gy = R[1], *Gz = R[2];
+        double* L = R[3];
+        const int variant = T->sl_variant;
+        const double p0 = T->sl_p0, p1 = T->sl_p1;
+        launch_n(p, s, [=] __device__(size_t i, double(&acc)[7]) {
+            const double n = den[i], gx = Gx[i], gy = Gy[i], gz = Gz[i];
+            const double sig = gx * gx + gy * gy + gz * gz, l = lap ? L[i] : 0.0;
+            double e, e_n, e_s, e_l;
+            semilocal_kinetic_point(n, sig, l, variant, p0, p1, e, e_n, e_s, e_l);
+            acc[0] += e - n * e_n - 2.0 * sig * e_s - l * e_l;
+            add_tensor(acc, -2.0 * e_s, gx, gy, gz);
+            if (lap) L[i] = e_l;
+        });
+        PAD_TRY(pad_stress_accumulate(p, s, gN, inv_n, inv_n, stress_out));
+        if (lap) {
+            PAD_TRY(pad_fft_forward(p, L, C[0], s));
+            PAD_TRY(pad_fft_forward(p, den, C[1], s));
+            const cufftDoubleComplex *El = C[0], *Nk = C[1];
+            launch_k(p, s, [=] __device__(size_t i, double(&acc)[7]) {
+                const KPoint k = make_kpoint(geom, (uint32_t)i);
+                const cufftDoubleComplex a = El[i], b = Nk[i];
+                const bool edge = k.j2 == 0 || (geom.e2 && k.j2 == geom.n2 / 2);
+                add_tensor(acc, 2.0 * (edge ? 1.0 : 2.0) * (a.x * b.x + a.y * b.y) * inv_n * inv_n, k.kx, k.ky, k.kz);
+            });
+            PAD_TRY(pad_stress_accumulate(p, s, gK, 0.0, 1.0, stress_out));
+        }
     }
     PAD_CUDA(cudaGetLastError());
     return PAD_OK;

@@ -78,3 +78,43 @@ __device__ __forceinline__ void pbe_point(double n, double sig, double c13, bool
         f_sig += n * dH_sig;
     }
 }
+
+// ---- semilocal kinetic functionals e(n, sigma, L), sigma = |grad n|^2, L = lap n ----------------------------------------
+//   e = C_TF n^(5/3) F(p, q),  p = s^2 = kSlC sigma / n^(8/3),  q = kSlC L / n^(5/3)   (functional_tools.py:122-135)
+//   LuoKarasievTrickey (PAD_SEMILOCAL_LKT, p0 = a):          F = 1 / cosh(a s) + (5/3) p
+//   PauliGaussian      (PAD_SEMILOCAL_PG, p0 = mu, p1 = beta): F = (5/3) p + exp(-mu p) + beta q^2
+//   e_n = C_TF n^(2/3) ((5/3) F - (8/3) p F_p - (5/3) q F_q),  e_sigma = C_TF kSlC F_p / n,  e_L = C_TF kSlC F_q
+// No guard on n: as in pbe_point, n <= 0 gives whatever these formulas give (cbrt of a negative density, a 0/0 at n = 0),
+// as the reference's torch expressions do; the densities the solvers produce are positive.
+constexpr double kSlC = 0.026121172985233605;      // (1/4)(3 pi^2)^(-2/3)
+
+// tanh(x) / x for x >= 0 (the sigma-derivative of 1/cosh(a s) carries tanh(a s) / s): its Taylor series below x = 1/16
+// (truncation error < 1e-14 relative), so sigma = 0 is no 0/0
+__device__ __forceinline__ double tanh_over_x_series(double x) {
+    const double x2 = x * x;
+    return 1.0 + x2 * (-1.0 / 3.0 + x2 * (2.0 / 15.0 + x2 * (-17.0 / 315.0 + x2 * (62.0 / 2835.0))));
+}
+
+__device__ __forceinline__ void semilocal_kinetic_point(double n, double sig, double lap, int variant, double p0, double p1,
+                                                        double& e, double& e_n, double& e_sig, double& e_lap) {
+    const double c13 = cbrt(n), n23 = c13 * c13, n53 = n * n23;
+    const double p = kSlC * sig / (n * n * n23);
+    double F, Fp, qFq = 0.0;
+    e_lap = 0.0;
+    if (variant == 0) {
+        const double s = sqrt(p), x = p0 * s;
+        const double sech = 1.0 / cosh(x);
+        const double tox = x < 0.0625 ? tanh_over_x_series(x) : tanh(x) / x;
+        F = sech + (5.0 / 3.0) * p;
+        Fp = 5.0 / 3.0 - 0.5 * p0 * p0 * sech * tox;
+    } else {
+        const double q = kSlC * lap / n53, g = exp(-p0 * p);
+        F = (5.0 / 3.0) * p + g + p1 * q * q;
+        Fp = 5.0 / 3.0 - p0 * g;
+        qFq = 2.0 * p1 * q * q;
+        e_lap = kCTF * kSlC * 2.0 * p1 * q;
+    }
+    e = kCTF * n53 * F;
+    e_n = kCTF * n23 * ((5.0 / 3.0) * F - (8.0 / 3.0) * p * Fp - (5.0 / 3.0) * qFq);
+    e_sig = kCTF * kSlC * Fp / n;
+}

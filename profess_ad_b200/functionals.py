@@ -272,6 +272,33 @@ class WangGovindCarter99(KineticFunctional):
         return _evaluate(box_vecs, den, launch).reshape(1)
 
 
+# Semilocal kinetic functionals T = int C_TF n^(5/3) F(p, q) with p = s^2 and q the reduced gradient / Laplacian of
+# functional_tools.py:122-135.  The constants are the published ones; they travel through the C ABI as arguments.
+LKT_A = 1.3                          # Luo, Karasiev, Trickey, PRB 98, 041111 (2018)
+PG_MU, PG_BETA = 40 / 27, 0.25       # PGSL0.25: Constantin, Fabiano, Della Sala, JPCL 9, 4385 (2018)
+
+
+def _launch_semilocal(variant, p0, p1):
+    def launch(plan, d, _, E, v, stream):
+        check(plan.lib.pad_eval_semilocal_kinetic(plan.handle, ptr(d), variant, p0, p1, ptr(E), ptr(v), 0, stream))
+    return launch
+
+
+_L_LKT = _launch_semilocal(_native.SEMILOCAL_LKT, LKT_A, 0.0)
+_L_PG = _launch_semilocal(_native.SEMILOCAL_PG, PG_MU, PG_BETA)
+
+
+def LuoKarasievTrickey(box_vecs, den):
+    """LKT (functionals.py:309): F = 1 / cosh(a s) + (5/3) s^2, a = 1.3.  8 FFTs."""
+    return _evaluate(box_vecs, den, _L_LKT)
+
+
+def PauliGaussian(box_vecs, den):
+    """Pauli-Gaussian PGSL0.25 (functionals.py:336): F = (5/3) p + exp(-mu p) + beta q^2, mu = 40/27, beta = 0.25.
+    10 FFTs: the Laplacian travels with the gradient."""
+    return _evaluate(box_vecs, den, _L_PG)
+
+
 # ----------------------------------------------------------------------------------------------
 #  exchange-correlation
 # ----------------------------------------------------------------------------------------------
@@ -332,6 +359,8 @@ pbe_exchange._pad_term = ('pbe', 1)
 pbe_correlation._pad_term = ('pbe', 2)
 PerdewBurkeErnzerhof._pad_term = ('pbe', 3)
 WangGovindCarter99._pad_term_of = lambda self, device=None: ('wgc99',) + self._args
+LuoKarasievTrickey._pad_term = ('semilocal', _native.SEMILOCAL_LKT, LKT_A, 0.0)
+PauliGaussian._pad_term = ('semilocal', _native.SEMILOCAL_PG, PG_MU, PG_BETA)
 
 
 # ----------------------------------------------------------------------------------------------
